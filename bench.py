@@ -23,6 +23,9 @@ SURVEY.md 8d), selected with --config:
            on the host cores, same metric/config, each step a bounded sample of the scan.
 
 Prints ONE JSON line on rank 0.
+
+  --dump-outputs DIR : after the timed steps, rank 0 writes what the last timed step returned (HtH, Htr, selected points, residual
+           sum) as float64 DIR/<name>.npy. The workload comes from fixed seeds, so two builds compare output for output.
 """
 from __future__ import annotations
 
@@ -410,7 +413,7 @@ def run_gpu(args, rank, world, local_rank):
                 if do_flush:
                     flush.fill_(i & 0xff)   # > L2 (126 MB): evicts the map between timed steps; outside the events
                 ev[i][0].record(stream)
-                fn()
+                res = fn()
                 ev[i][1].record(stream)
                 a, b = g.last_pass_kernel_times()
                 knn_ms.append(a)
@@ -422,11 +425,13 @@ def run_gpu(args, rank, world, local_rank):
             l1 = g.launch_count()
         ms = [a.elapsed_time(b) for a, b in ev]
         timed.last_steps = ms
+        timed.last_result = res
         return float(np.sum(ms)), (l1 - l0), float(np.mean(knn_ms)), float(np.mean(plane_ms))
 
     sampler.recording.set()               # samples across all timed loops (each lasts only a few ms)
     tot_ms, launches, knn_ms, plane_ms = timed(step_resident, args.steps, args.warmup, True)
     step_ms = list(timed.last_steps)
+    last_step = timed.last_result
     warm_ms, _, knn_warm, plane_warm = timed(step_resident, args.steps, 1, False)
     e2e_ms, _, e2e_knn_ms, e2e_plane_ms = timed(step_e2e, args.steps, args.warmup, True)
     e2e_staged_ms, _, _, _ = timed(step_e2e_staged, args.steps, args.warmup, True)
@@ -560,11 +565,22 @@ def run_gpu(args, rank, world, local_rank):
                 out["cpu_baseline"]["value_mp_proc_num_3"] = r3["n"] / float(np.median(r3["times"]))
         except Exception as e:  # the oracle is test infrastructure; its absence must not hide the GPU number
             out["cpu_baseline"] = {"value": None, "unit": UNIT, "cores": threads, "kind": "unavailable", "sample": repr(e)}
+    if rank == 0 and args.dump_outputs:
+        H, b, m, rs = last_step
+        dump_outputs(args.dump_outputs, {"HtH": H, "Htr": b, "selected_points": m, "residual_sum": rs})
     if rank == 0:
         emit(out)
     g.close()
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: what the last timed step returned, one float64 <name>.npy each. The workload is generated from fixed seeds, so
+    two builds run with the same arguments can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, np.float64))
 
 
 def main():
@@ -588,7 +604,13 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=240_000)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-bind", action="store_true", help="do not bind the launch thread / pinned frame to the GPU's NUMA node")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (HtH, Htr, selected points, residual sum) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours: the reference arm sizes its scan sample by its own speed, so its outputs vary run to run")
     args.scan_points = args.scan_points or CONFIGS[args.config][0]
     args.map_points = args.map_points or CONFIGS[args.config][1]
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup

@@ -1,8 +1,9 @@
-"""Generate tests/golden/*.npz: inputs + outputs of the hot path computed HERE with the reference's verbatim
-ikd-Tree (oracle/_ref, backend 1) and the restated measurement model. The fixtures travel to the GPU box,
-where /root/reference does not exist; tests compare both the oracle and the CUDA path against them.
+"""Generate tests/golden/*.npz: inputs + outputs of the hot path computed with the reference's verbatim
+ikd-Tree (oracle/_ref, backend 1) and the restated measurement model, plus (ikd_tree.npz) the verbatim tree's
+answers to the oracle checks of tests/ikd_cases.py. Tests compare both the oracle and the CUDA path against
+them, so they need no copy of the reference where they run.
 
-Run from the repo root in the build container:  python tools/make_golden.py
+Needs oracle/_ref (make -C oracle ref REF=<checkout of the reference>). Run from the repo root:  python tools/make_golden.py  (all files) or  python tools/make_golden.py ikd_tree  (that one only)
 """
 import os
 import sys
@@ -11,6 +12,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+import ikd_cases  # noqa: E402
 from lidar_imu_init_b200 import scenes  # noqa: E402
 from oracle import oracle as orc  # noqa: E402
 
@@ -50,7 +53,34 @@ def one(name, cfg, imu_en):
     print(name, "m", m, m2, "add", na, nn, "live", len(live))
 
 
+def ikd_tree():
+    assert orc.has_ikd(), "golden vectors must come from the verbatim ikd-Tree build (make -C oracle ref)"
+    c, q = ikd_cases.knn_case()
+    om = orc.OracleMap(c["ds"], 1)
+    om.build(c["map_xyz"])
+    x, d2, cnt, _ = om.knn(q)
+    out = dict(knn_inputs=ikd_cases.digest(c["map_xyz"], q), knn_nbr=ikd_cases.map_rows(x, cnt, c["map_xyz"]), knn_d2=d2, knn_cnt=cnt)
+    ds, mp, batches = ikd_cases.add_points_case()
+    om = orc.OracleMap(ds, 1)
+    om.build(mp)
+    for b, down in batches:
+        om.add_points(b, down)
+    cand = ikd_cases.add_points_candidates(mp, batches)
+    out.update(add_inputs=ikd_cases.digest(cand), add_validnum=np.int32(om.validnum()), add_live=ikd_cases.live_mask(om.flatten(), cand))
+    pts, boxes = ikd_cases.delete_boxes_case()
+    om = orc.OracleMap(0.15, 1)
+    om.build(pts)
+    d = om.delete_boxes(boxes)
+    out.update(del_inputs=ikd_cases.digest(pts, boxes), del_deleted=np.int32(d), del_validnum=np.int32(om.validnum()),
+               del_live=ikd_cases.live_mask(om.flatten(), pts))
+    np.savez_compressed(ikd_cases.GOLD, **out)
+    print("ikd_tree", "knn", int((cnt == 5).sum()), "add live", out["add_validnum"], "deleted", d)
+
+
 if __name__ == "__main__":
+    if sys.argv[1:] == ["ikd_tree"]:
+        ikd_tree()
+        sys.exit(0)
     one("c1_lo", scenes.make_config("C1", imu_en=False), False)
     one("c1_lio", scenes.make_config("C1", imu_en=True), True)
     one("c2small_lo", scenes.make_config("C2", N=3000, M=40000, open_air_frac=0.02, imu_en=False), False)

@@ -83,6 +83,27 @@ int liinit_map_download(liinit_ctx* h, float* xyz, int cap_points, int* n);
  * squared distance <= max_dist (sic). k must be 5. out_xyz [n*5*3], out_d2 [n*5] (-1 where missing), out_cnt [n]. */
 int liinit_map_nearest_search(liinit_ctx* h, const float* q_xyz, int stride_floats, int n, double max_dist,
                               float* out_xyz, float* out_d2, int* out_cnt);
+/* KD_TREE::Nearest_Search(point, k, Nearest_Points, Point_Distance, max_dist) (ikd_Tree.cpp:349-379,825-968) for n world-frame
+ * queries, any 1 <= k <= LIINIT_KNN_MAX_K and max_dist >= 0 or +INFINITY (the reference's default, ikd_Tree.h:176).
+ * out_xyz [n*k*3], out_d2 [n*k], out_cnt [n]: per query the count found, then that many neighbours ascending in PointType_CMP order
+ * (ikd_Tree.h:57-60: distances within 1e-10 go by ascending x); d2 = -1 and xyz = 0 past the count.
+ *   - d2 is fp32 (dx*dx + dy*dy) + dz*dz without FMA (ikd_Tree.cpp:1273-1277); a point qualifies when d2 <= max_dist (sic, :842),
+ *     the float d2 compared with the double max_dist, i.e. with the largest float not above it.
+ *   - For max_dist >= 1 or +INFINITY the answer is the exact k nearest live points under that test: the reference's box prune at
+ *     max_dist^2 (:827-828) never removes such a point. For 0 <= max_dist < 1 the reference's answer depends on the shape of its
+ *     tree; this search applies the point test alone (DESIGN.md section 4, deviations).
+ *   - Which of several points tied at exactly the k-th distance is returned is not specified.
+ *   - An empty map, a query with a non-finite coordinate or no point within max_dist gives a count of 0. A query far from the map --
+ *     also beyond the range brick keys can pack -- still gets its k nearest points when max_dist allows.
+ * LIINIT_ERR_INVALID (the context stays usable) for k outside 1..LIINIT_KNN_MAX_K, max_dist NaN or negative, a null pointer, n < 0,
+ * or a stride other than 3, 4 or 12. liinit_map_nearest_search and the ICP pass do not use this search. */
+#define LIINIT_KNN_MAX_K 32
+int liinit_map_knn_search(liinit_ctx* h, const float* q_xyz, int stride_floats, int n, int k, double max_dist,
+                          float* out_xyz, float* out_d2, int* out_cnt);
+/* Same search with device pointers (queries, outputs), queued on the context's stream with no host synchronisation (as
+ * liinit_icp_iterate_device). The host form stages its queries through this one. */
+int liinit_map_knn_search_device(liinit_ctx* h, const float* d_q_xyz, int stride_floats, int n, int k, double max_dist,
+                                 float* d_out_xyz, float* d_out_d2, int* d_out_cnt);
 
 /* per-scan hot path (replaces laserMapping.cpp:936-1080) ---------------------------- */
 /* feats_down_body (laserMapping.cpp:917-919): once per scan; resets selection flags / neighbour lists. */
@@ -162,6 +183,7 @@ int liinit_debug_esti_plane(liinit_ctx* h, const float* nb_xyz, int n, double* p
  * buffer, a system-scope flag, a spin on the other ranks' flags, a rank-ordered sum (bit-identical on every rank): no extra launch, no
  * NCCL kernel. If any rank cannot map its peers (ranks as threads of one process, no peer access) or LIINIT_COMM_MODE=nccl is set, all
  * ranks use ncclAllReduce on the context's stream instead. NCCL always carries the set-up and the all-gathers of per-point results.
+ * liinit_map_knn_search / _device are rank-local: each rank answers from its own replica of the map, with no collective.
  * As with any collective: a rank that does not make the call (it returned an error earlier, or died) leaves the others waiting -- the
  * spin in the plane kernel has no time-out, exactly like a pending ncclAllReduce; supervise the ranks from outside. */
 #define LIINIT_COMM_ID_BYTES 128

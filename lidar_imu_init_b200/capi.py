@@ -33,7 +33,7 @@ _i32 = np.ctypeslib.ndpointer(dtype=np.int32, flags="C_CONTIGUOUS")
 
 SYMBOLS = [
     "liinit_create", "liinit_destroy", "liinit_last_error", "liinit_set_stream", "liinit_map_build", "liinit_map_add_points", "liinit_map_delete_boxes",
-    "liinit_map_compact", "liinit_map_validnum", "liinit_map_size", "liinit_map_download", "liinit_map_nearest_search", "liinit_scan_upload", "liinit_scan_attach_host", "liinit_scan_upload_raw", "liinit_scan_download_body", "liinit_raw_upload", "liinit_raw_undistort_cv", "liinit_raw_undistort_imu",
+    "liinit_map_compact", "liinit_map_validnum", "liinit_map_size", "liinit_map_download", "liinit_map_nearest_search", "liinit_map_knn_search", "liinit_map_knn_search_device", "liinit_scan_upload", "liinit_scan_attach_host", "liinit_scan_upload_raw", "liinit_scan_download_body", "liinit_raw_upload", "liinit_raw_undistort_cv", "liinit_raw_undistort_imu",
     "liinit_raw_download", "liinit_raw_downsample",
     "liinit_icp_iterate", "liinit_icp_iterate_device", "liinit_scan_download_effect", "liinit_scan_download_state",
     "liinit_map_incremental", "liinit_last_pass_timing", "liinit_last_pass_kernel_times", "liinit_launch_count", "liinit_map_stats", "liinit_knn_index",
@@ -70,6 +70,8 @@ def load():
     L.liinit_map_size.argtypes = [vp, C.POINTER(C.c_int)]
     L.liinit_map_download.argtypes = [vp, vp, C.c_int, C.POINTER(C.c_int)]
     L.liinit_map_nearest_search.argtypes = [vp, vp, C.c_int, C.c_int, C.c_double, vp, vp, vp]
+    L.liinit_map_knn_search.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, C.c_double, vp, vp, vp]
+    L.liinit_map_knn_search_device.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, C.c_double, vp, vp, vp]
     L.liinit_scan_upload.argtypes = [vp, vp, C.c_int, C.c_int]
     L.liinit_scan_attach_host.argtypes = [vp, vp, C.c_int, C.c_int]
     L.liinit_scan_upload_raw.argtypes = [vp, vp, C.c_int, C.c_int, C.c_float, C.POINTER(C.c_int)]
@@ -200,6 +202,21 @@ class LiInitGpu:
         cnt = np.zeros(n, np.int32)
         self._ck(self.L.liinit_map_nearest_search(self.h, _ptr(a), a.shape[1], n, max_dist, _ptr(xyz), _ptr(d2), _ptr(cnt)))
         return xyz, d2, cnt
+
+    def knn_search(self, q, k, max_dist=float("inf")):
+        """KD_TREE::Nearest_Search(q, k, ..., max_dist) for every row of q -> (xyz [n,k,3], d2 [n,k], cnt [n]); -1 / zeros past cnt"""
+        a = _pts(q)
+        n = a.shape[0]
+        xyz = np.zeros((n, k, 3), np.float32)
+        d2 = np.zeros((n, k), np.float32)
+        cnt = np.zeros(n, np.int32)
+        self._ck(self.L.liinit_map_knn_search(self.h, _ptr(a), a.shape[1], n, int(k), float(max_dist), _ptr(xyz), _ptr(d2), _ptr(cnt)))
+        return xyz, d2, cnt
+
+    def knn_search_device(self, q_ptr: int, stride: int, n: int, k: int, max_dist: float, out_xyz_ptr: int, out_d2_ptr: int, out_cnt_ptr: int):
+        """The same search on device memory (e.g. data_ptr() of CUDA torch tensors), queued on the context's stream, no synchronisation"""
+        self._ck(self.L.liinit_map_knn_search_device(self.h, C.c_void_p(q_ptr), int(stride), int(n), int(k), float(max_dist), C.c_void_p(out_xyz_ptr),
+                                                     C.c_void_p(out_d2_ptr), C.c_void_p(out_cnt_ptr)))
 
     # ---- scan ----
     def scan_upload(self, body):

@@ -37,12 +37,14 @@ public:
     // KD_TREE::size / validnum (ikd_Tree.cpp:71-88,120-137)
     int size() { int n = 0; ck(liinit_map_size(h_, &n)); return n; }
     int validnum() { int n = 0; ck(liinit_map_validnum(h_, &n)); return n; }
-    // KD_TREE::Nearest_Search(point, 5, Nearest_Points, Point_Distance, 5) (ikd_Tree.cpp:349-379) for one query
+    // KD_TREE::Nearest_Search(point, k, Nearest_Points, Point_Distance, max_dist) (ikd_Tree.cpp:349-379) for one query, 1 <= k <= 32.
+    // k = 5 with max_dist = 5 (the node's call, laserMapping.cpp:980) takes the path of the ICP pass; any other k / max_dist the general
+    // search (liinit_map_knn_search). The reference's default max_dist is INFINITY (ikd_Tree.h:176); this one stays 5 for existing callers.
     void Nearest_Search(const PointT& p, int k, PointVector& near, std::vector<float>& d2, double max_dist = 5.0) {
-        if (k != LIINIT_NUM_MATCH_POINTS) throw std::invalid_argument("k must be 5");
-        float q[3] = {p.x, p.y, p.z}, xyz[15], dd[5];
+        float q[3] = {p.x, p.y, p.z}, xyz[3 * LIINIT_KNN_MAX_K], dd[LIINIT_KNN_MAX_K];
         int cnt = 0;
-        ck(liinit_map_nearest_search(h_, q, 3, 1, max_dist, xyz, dd, &cnt));
+        if (k == LIINIT_NUM_MATCH_POINTS && max_dist == 5.0) ck(liinit_map_nearest_search(h_, q, 3, 1, max_dist, xyz, dd, &cnt));
+        else ck(liinit_map_knn_search(h_, q, 3, 1, k, max_dist, xyz, dd, &cnt));
         near.assign(cnt, PointT());
         d2.assign(dd, dd + cnt);
         for (int j = 0; j < cnt; j++) { near[j].x = xyz[3 * j]; near[j].y = xyz[3 * j + 1]; near[j].z = xyz[3 * j + 2]; }

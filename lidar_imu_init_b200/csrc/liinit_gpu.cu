@@ -20,6 +20,7 @@
 #include "common.cuh"
 #include "icp_kernels.cuh"
 #include "knn_kernels.cuh"
+#include "knn_general.cuh"
 #include "cells.cuh"
 #include "map_kernels.cuh"
 #include "voxelgrid_kernels.cuh"
@@ -80,6 +81,17 @@ NcclApi* nccl_api() {
     return &api;
 }
 #endif
+
+// device scratch (per call, or owned by the context) that is released on every return path (the CU() macro returns early on a CUDA error)
+template <class T>
+struct DevBuf {
+    T* p = nullptr;
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    ~DevBuf() { if (p) cudaFree(p); }
+    cudaError_t alloc(size_t count) { return cudaMalloc(&p, count * sizeof(T)); }
+};
 
 struct Ctx {
     liinit_config cfg;
@@ -158,6 +170,12 @@ struct Ctx {
     int max_blocks = 0;
     // knn query scratch
     float* d_q_d2 = nullptr;
+    // k-NN search for any k / max_dist (knn_general.cuh): copies of the map's brick entries, walked by far / unbounded queries;
+    // rebuilt on the stream when map_version moved since
+    unsigned map_version = 0;      // bumped by every call that changes the map
+    DevBuf<uint4> knn_occ;         // [hash_slots] (a brick per hash slot at most), allocated on first use
+    unsigned knn_occ_version = 0;
+    bool knn_occ_valid = false;
     // stats
     long long launches = 0;
     float last_ms = 0.f;
@@ -181,17 +199,6 @@ struct Ctx {
     } while (0)
 
 inline int nblk(long long n, int t) { return (int)((n + t - 1) / t); }
-
-// per-call device scratch that is released on every return path (the CU() macro returns early on a CUDA error)
-template <class T>
-struct DevBuf {
-    T* p = nullptr;
-    DevBuf() = default;
-    DevBuf(const DevBuf&) = delete;
-    DevBuf& operator=(const DevBuf&) = delete;
-    ~DevBuf() { if (p) cudaFree(p); }
-    cudaError_t alloc(size_t count) { return cudaMalloc(&p, count * sizeof(T)); }
-};
 
 int fail(Ctx* c, int code, const std::string& msg) {
     c->err = msg;
@@ -781,6 +788,7 @@ int liinit_map_build(liinit_ctx* h, const float* xyz, int stride, int n) {
     CU(cudaSetDevice(c->device));
     if (n > c->cfg.max_map_points) return fail(c, LIINIT_ERR_CAPACITY, "n exceeds max_map_points");
     c->map_epoch++;
+    c->map_version++;
     // KD_TREE::Build replaces the tree (ikd_Tree.cpp:337-339)
     CU(cudaMemsetAsync(c->d_counters, 0, sizeof(int) * CNT_COUNT, c->stream));
     CU(cudaMemsetAsync(c->M.pool_top, 0, sizeof(unsigned long long), c->stream));
@@ -813,6 +821,7 @@ namespace {
 // points, clear hash + pool, re-insert them (the Build path): every brick gets one tight slab, empty bricks disappear.
 int compact_map(Ctx* c) {
     c->map_epoch++;
+    c->map_version++;
     int r = fetch_counters(c);
     if (r) return r;
     const int live = c->h_counters[CNT_LIVE];
@@ -872,6 +881,7 @@ int liinit_map_add_points(liinit_ctx* h, const float* xyz, int stride, int n, in
     Ctx* c = &h->c;
     CU(cudaSetDevice(c->device));
     c->map_epoch++;
+    c->map_version++;
     {
         int r = maybe_compact(c, n);
         if (r) return r;
@@ -900,6 +910,7 @@ int liinit_map_delete_boxes(liinit_ctx* h, const float* boxes, int nbox, int* de
     if (deleted) *deleted = 0;
     if (nbox == 0) return LIINIT_OK;
     c->map_epoch++;
+    c->map_version++;
     if ((size_t)nbox * 6 > c->stage_raw_floats) return fail(c, LIINIT_ERR_CAPACITY, "too many boxes");
     CU(cudaMemcpyAsync(c->d_stage_raw, boxes, (size_t)nbox * 6 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemsetAsync(c->d_vg_misc + 6, 0, sizeof(int), c->stream));
@@ -1031,6 +1042,87 @@ int liinit_map_nearest_search(liinit_ctx* h, const float* q, int stride, int n, 
                     }
                 }
         }
+    }
+    return LIINIT_OK;
+}
+
+}  // extern "C"
+
+namespace {
+// The reference compares the float d2 with the double max_dist (ikd_Tree.cpp:842): d2 <= max_dist <=> d2 <= the largest float not above
+// max_dist. (float)max_dist rounds to nearest and would admit points the reference rejects whenever max_dist is not a float.
+float float_at_most(double v) {
+    float f = (float)v;
+    if ((double)f > v) f = std::nextafter(f, -INFINITY);
+    return f;
+}
+
+int knn_args_check(Ctx* c, int stride, int n, int k, double max_dist) {
+    if (k < 1 || k > LIINIT_KNN_MAX_K) return fail(c, LIINIT_ERR_INVALID, "k must be in 1.." + std::to_string(LIINIT_KNN_MAX_K));
+    if (!(max_dist >= 0.0)) return fail(c, LIINIT_ERR_INVALID, "max_dist must be >= 0 or +INFINITY (not NaN)");
+    if (n < 0) return fail(c, LIINIT_ERR_INVALID, "n must be >= 0");
+    if (stride != 3 && stride != 4 && stride != 12) return fail(c, LIINIT_ERR_INVALID, "stride_floats must be 3, 4 or 12");
+    return LIINIT_OK;
+}
+
+// The search itself, queued on the context's stream: queries and outputs are device memory.
+int knn_general(Ctx* c, const float* d_q, int stride, int n, int k, double max_dist, float* d_xyz, float* d_d2, int* d_cnt) {
+    if (n == 0) return LIINIT_OK;
+    if (!c->knn_occ.p) CU(c->knn_occ.alloc(c->hash_slots));
+    if (!c->knn_occ_valid || c->knn_occ_version != c->map_version) {
+        k_knn_occ_build<<<c->num_sms * 4, 256, 0, c->stream>>>(c->M, c->knn_occ.p);
+        c->launches++;
+        c->knn_occ_version = c->map_version;
+        c->knn_occ_valid = true;
+    }
+    const int wpb = LI_KNN_GEN_THREADS / 32;
+    long long grid = ((long long)n + wpb - 1) / wpb;
+    if (grid > c->max_blocks) grid = c->max_blocks;
+    k_knn_general<<<(int)grid, LI_KNN_GEN_THREADS, 0, c->stream>>>(c->M, c->knn_occ.p, d_q, stride, n, k, float_at_most(max_dist), c->rho2, d_xyz, d_d2,
+                                                                   d_cnt);
+    c->launches++;
+    CU(cudaGetLastError());
+    return LIINIT_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int liinit_map_knn_search_device(liinit_ctx* h, const float* d_q, int stride, int n, int k, double max_dist, float* d_out_xyz, float* d_out_d2,
+                                 int* d_out_cnt) {
+    if (!h) return LIINIT_ERR_INVALID;
+    Ctx* c = &h->c;
+    if ((n > 0 && (!d_q || !d_out_xyz || !d_out_d2 || !d_out_cnt))) return fail(c, LIINIT_ERR_INVALID, "null pointer");
+    int r = knn_args_check(c, stride, n, k, max_dist);
+    if (r) return r;
+    CU(cudaSetDevice(c->device));
+    return knn_general(c, d_q, stride, n, k, max_dist, d_out_xyz, d_out_d2, d_out_cnt);
+}
+
+int liinit_map_knn_search(liinit_ctx* h, const float* q, int stride, int n, int k, double max_dist, float* out_xyz, float* out_d2, int* out_cnt) {
+    if (!h) return LIINIT_ERR_INVALID;
+    Ctx* c = &h->c;
+    if (n > 0 && (!q || !out_xyz || !out_d2 || !out_cnt)) return fail(c, LIINIT_ERR_INVALID, "null pointer");
+    int r = knn_args_check(c, stride, n, k, max_dist);
+    if (r) return r;
+    CU(cudaSetDevice(c->device));
+    if (n == 0) return LIINIT_OK;
+    const int chunk = n < c->stage_pts_cap ? n : c->stage_pts_cap;
+    DevBuf<float> bxyz, bd2;
+    DevBuf<int> bcnt;
+    CU(bxyz.alloc((size_t)chunk * k * 3));
+    CU(bd2.alloc((size_t)chunk * k));
+    CU(bcnt.alloc((size_t)chunk));
+    for (long long off = 0; off < n; off += c->stage_pts_cap) {
+        const int m = (int)((n - off < c->stage_pts_cap) ? (n - off) : c->stage_pts_cap);
+        r = stage_points(c, q + (size_t)off * stride, stride, m);
+        if (r) return r;
+        r = knn_general(c, reinterpret_cast<const float*>(c->d_stage_pts), 4, m, k, max_dist, bxyz.p, bd2.p, bcnt.p);
+        if (r) return r;
+        CU(cudaMemcpyAsync(out_xyz + (size_t)off * k * 3, bxyz.p, (size_t)m * k * 3 * 4, cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaMemcpyAsync(out_d2 + (size_t)off * k, bd2.p, (size_t)m * k * 4, cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaMemcpyAsync(out_cnt + off, bcnt.p, (size_t)m * 4, cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaStreamSynchronize(c->stream));   // the staging buffer is reused by the next chunk
     }
     return LIINIT_OK;
 }
@@ -1347,6 +1439,7 @@ int liinit_map_incremental(liinit_ctx* h, const double* R, const double* p, cons
         if (r) return r;
     }
     c->map_epoch++;
+    c->map_version++;
     {
         int r = maybe_compact(c, n);
         if (r) return r;

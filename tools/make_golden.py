@@ -3,7 +3,7 @@ ikd-Tree (oracle/_ref, backend 1) and the restated measurement model, plus (ikd_
 answers to the oracle checks of tests/ikd_cases.py. Tests compare both the oracle and the CUDA path against
 them, so they need no copy of the reference where they run.
 
-Needs oracle/_ref (make -C oracle ref REF=<checkout of the reference>). Run from the repo root:  python tools/make_golden.py  (all files) or  python tools/make_golden.py ikd_tree  (that one only)
+Needs oracle/_ref (make -C oracle ref REF=<checkout of the reference>). Run from the repo root:  python tools/make_golden.py  (all files) or  python tools/make_golden.py ikd_tree | ikd_knn  (that one only)
 """
 import os
 import sys
@@ -14,6 +14,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 import ikd_cases  # noqa: E402
+import knn_general_cases  # noqa: E402
 from lidar_imu_init_b200 import scenes  # noqa: E402
 from oracle import oracle as orc  # noqa: E402
 
@@ -77,9 +78,44 @@ def ikd_tree():
     print("ikd_tree", "knn", int((cnt == 5).sum()), "add live", out["add_validnum"], "deleted", d)
 
 
+def ikd_knn():
+    """The verbatim tree's KD_TREE::Nearest_Search(q, k, ..., max_dist) over the grid of tests/knn_general_cases.py (oracle/_ref/libikd_ref.so: the
+    tree alone, any k)"""
+    import ctypes as C
+    lib = os.path.join(ROOT, "oracle", "_ref", "libikd_ref.so")
+    assert os.path.exists(lib), "golden vectors must come from the verbatim ikd-Tree build (make -C oracle ref)"
+    L = C.CDLL(lib)
+    L.ikdref_create.restype = C.c_void_p
+    L.ikdref_create.argtypes = [C.c_float]
+    L.ikdref_destroy.argtypes = [C.c_void_p]
+    L.ikdref_build.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
+    L.ikdref_nearest.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
+    c, q = knn_general_cases.knn_general_case()
+    mp = np.ascontiguousarray(c["map_xyz"], np.float32)
+    q = np.ascontiguousarray(q, np.float32)
+    t = L.ikdref_create(float(c["ds"]))
+    L.ikdref_build(t, mp.ctypes.data, len(mp))
+    out = dict(inputs=ikd_cases.digest(mp, q))
+    for k in knn_general_cases.KNN_KS:
+        for md in knn_general_cases.KNN_MAX_DISTS:
+            xyz = np.zeros((len(q), k, 3), np.float32)
+            d2 = np.zeros((len(q), k), np.float32)
+            cnt = np.zeros(len(q), np.int32)
+            L.ikdref_nearest(t, q.ctypes.data, len(q), k, md, xyz.ctypes.data, d2.ctypes.data, cnt.ctypes.data, 8)
+            out[f"cnt_k{k}_{md}"] = cnt
+            out[f"nbr_k{k}_{md}"] = ikd_cases.map_rows(xyz, cnt, mp).astype(np.int16)
+            print("k", k, "max_dist", md, "found", int(cnt.sum()))
+    L.ikdref_destroy(t)
+    np.savez_compressed(knn_general_cases.GOLD_KNN, **out)
+    print("ikd_knn", os.path.getsize(knn_general_cases.GOLD_KNN), "bytes")
+
+
 if __name__ == "__main__":
     if sys.argv[1:] == ["ikd_tree"]:
         ikd_tree()
+        sys.exit(0)
+    if sys.argv[1:] == ["ikd_knn"]:
+        ikd_knn()
         sys.exit(0)
     one("c1_lo", scenes.make_config("C1", imu_en=False), False)
     one("c1_lio", scenes.make_config("C1", imu_en=True), True)
